@@ -20,15 +20,19 @@ c2     = second workload on the same line (BASELINE.json configs[1]): WHERE leve
 --impl reference: the declared CPU stand-in for the reference's DataFusion path (BASELINE.md §3):
          pyarrow/Acero, all host threads, same files, same query, on rank 0's shard.
 
-Launch: python bench.py [--gpus N --steps K --warmup W]; under torchrun one rank per GPU.
+Launch: python bench.py [--gpus N --steps K --warmup W] [--dump-outputs DIR]; under torchrun one rank per GPU.
+--steps K is the number of timed steps of every timed loop (resident, e2e, C2, reference arm).
+--dump-outputs DIR: rank 0 writes what the last timed steps returned, as float64 .npy files (see dump_outputs).
 """
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -38,7 +42,9 @@ sys.path.insert(0, ROOT)
 ROW_GROUP = 262_144
 RGS_PER_FILE = 16                  # one Parquet file per ingest minute batch in Parseable
 RGS_PER_GPU = 480                  # 125 829 120 rows per GPU; 8 GPUs: 1 006 632 960 rows ("1B")
-DATA_DIR = os.environ.get("PQB_DATA_DIR", "/tmp/pqb_bench")
+# the generated tables are cached between runs, one directory per user: on a shared host another user's directory is
+# neither writable nor known to hold complete files
+DATA_DIR = os.environ.get("PQB_DATA_DIR") or os.path.join(tempfile.gettempdir(), f"pqb_bench_{os.getuid()}")
 # the columns the two workloads reference (logs16 has 16; an unreferenced column is never read by either arm)
 COLS = ["p_timestamp", "level", "latency_ms", "host", "bytes", "status", "duration_s", "cpu"]
 C4_COLS = ["p_timestamp", "host", "status", "bytes", "latency_ms", "duration_s", "cpu"]
@@ -102,6 +108,7 @@ class ClockSampler:
         try:
             self.proc = subprocess.Popen(["nvidia-smi", f"--query-gpu={q}", "--format=csv,noheader,nounits", "-i", str(self.idx), "-lms", "10"],
                                          stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self._terminate)          # a run that fails before stop() must not leave the sampler running
             self.t = threading.Thread(target=self._read, daemon=True)
             self.t.start()
         except Exception:
@@ -114,15 +121,20 @@ class ClockSampler:
     def window(self, t0, t1):
         self.windows.append((t0, t1))
 
+    def _terminate(self):
+        if self.proc and self.proc.poll() is None:
+            self.proc.terminate()
+            try:
+                self.proc.wait(timeout=2)
+            except Exception:
+                self.proc.kill()
+                self.proc.wait()
+
     def stop(self) -> dict:
         if not self.proc:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"], "samples": 0}
         time.sleep(0.05)
-        self.proc.terminate()
-        try:
-            self.proc.wait(timeout=2)
-        except Exception:
-            self.proc.kill()
+        self._terminate()
         # a sample describes the ~10 ms before it was printed
         inside = [r for (t, r) in self.rows if any(a <= t <= b + 0.03 for a, b in self.windows)]
         sm = sorted(int(r[0]) for r in inside if r and r[0].isdigit())
@@ -186,6 +198,44 @@ def tables_agree(a, b, what: str):
         else:
             assert x.equals(y), f"{what}: column {name} differs"
     return True
+
+
+DUMP_BYTES = 64_000_000            # all arrays of one --dump-outputs directory together
+DUMP_SEED = 20260922
+
+
+def _utf8_codes(arr):
+    """Utf8 values as float64: the top 53 bits of a BLAKE2b digest of the UTF-8 bytes (a float64 holds such an integer
+    exactly), NaN for NULL. Equal strings give equal codes, so two builds' key columns compare as numbers."""
+    import hashlib
+    import numpy as np
+    return np.array([np.nan if v is None else float(int.from_bytes(hashlib.blake2b(v.encode(), digest_size=8).digest(), "little") >> 11)
+                     for v in arr.to_pylist()], dtype=np.float64)
+
+
+def dump_outputs(out_dir: str, c4_table, c2_ids) -> dict:
+    """Write what the last timed steps returned as out_dir/<name>.npy, float64 (integers are exact below 2**53, NULL is NaN):
+    c4_<column>: the C4 result table in canonical order (canon: sorted by host, status), host as _utf8_codes;
+    c2_row_ids: the C2 row ids as returned (ascending); when they do not fit in DUMP_BYTES next to the C4 arrays, a sample
+    at positions drawn with DUMP_SEED, kept in order.  The tables are the seeded ones ensure_data writes, so two builds run
+    with the same arguments can be compared array for array.  Returns {name: length}."""
+    import numpy as np
+    arrays = {}
+    t = canon(c4_table)
+    for name, short in zip(C4_NAMES, ["host", "status", "count", "sum_bytes", "min_latency_ms", "max_latency_ms",
+                                      "sum_duration_s", "max_cpu"]):
+        c = t[name]
+        arrays["c4_" + short] = _utf8_codes(c) if name == "host" else np.asarray(c.to_numpy(zero_copy_only=False), dtype=np.float64)
+    if c2_ids is not None:
+        room = (DUMP_BYTES - sum(a.nbytes + 128 for a in arrays.values()) - 128) // 8     # 128: the .npy header
+        if len(c2_ids) > room:
+            keep = np.sort(np.random.default_rng(DUMP_SEED).choice(len(c2_ids), size=room, replace=False))
+            c2_ids = c2_ids[keep]
+        arrays["c2_row_ids"] = c2_ids.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return {name: len(a) for name, a in arrays.items()}
 
 
 def plain_schema():
@@ -258,14 +308,13 @@ def run_reference(args, rank: int, world: int):
     pa.set_cpu_count(cores)
     pa.set_io_thread_count(cores)
     vals = []
-    t_start = time.time()
     acero_groupby(shard, nrg)                             # warm: page cache, thread pools
-    while len(vals) < max(1, args.steps):
+    for _ in range(args.steps):
         t = time.time()
-        _, rows = acero_groupby(shard, nrg)
+        g, rows = acero_groupby(shard, nrg)
         vals.append((rows / (time.time() - t), rows, time.time() - t))
-        if len(vals) >= 5 and time.time() - t_start > 150.0:
-            break
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, g, None)
     vs = sorted(v[0] for v in vals)
     v = vs[len(vs) // 2]                                  # median
     ms = 1000.0 * sorted(x[2] for x in vals)[len(vals) // 2]
@@ -311,14 +360,17 @@ def pin_to_gpu_numa(local_rank: int) -> dict:
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=30)
+    ap.add_argument("--steps", type=int, default=30, help="timed steps of every timed loop")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--row-groups", type=int, default=RGS_PER_GPU, help="row groups PER GPU (smaller tables for development runs)")
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--skip-e2e", action="store_true")
     ap.add_argument("--skip-c2", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed steps to DIR/<name>.npy (dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -444,7 +496,8 @@ def main():
     value = rows_per_gpu * world / (dt / args.steps)
     algo_bytes = r.metrics["algorithmic_bytes"]
     d2h_res = r.metrics["d2h_bytes"]
-    assert r.table().num_rows == groups
+    c4_last = r.table()                                # the last timed step's answer (--dump-outputs)
+    assert c4_last.num_rows == groups
     if rank == 0:
         print(f"[bench] C4 resident step: wall {ms_per_step:.3f} ms = pq_query_open {sum(host_ms) / len(host_ms):.3f} ms (device {sum(dev_ms) / len(dev_ms):.3f} ms, "
               f"scan kernels {sum(scan_ms) / len(scan_ms):.3f} ms, all-reduce {sum(ar_ms) / len(ar_ms):.3f} ms) + binding/Arrow import; table open {open_s:.2f} s",
@@ -466,7 +519,7 @@ def main():
         for _ in range(2):
             re_ = prov_e.aggregate(keys, aggs, tf, flags=ar_flag)
         barrier()
-        k = max(3, min(args.steps, 6))
+        k = args.steps
         t_a = time.perf_counter()
         for _ in range(k):
             re_ = prov_e.aggregate(keys, aggs, tf, flags=ar_flag)
@@ -485,6 +538,7 @@ def main():
 
     # ================= second workload: C2 scan + filter =================
     c2 = None
+    c2_last_ids = None
     if not args.skip_c2:
         flt = c2_filters() + tf
         tbl2 = DeviceTable(files, C2_COLS)
@@ -518,6 +572,8 @@ def main():
         clocks.window(t_a, t_b)
         dt2 = max_over_ranks(t_b - t_a)
         launches += l2
+        if args.dump_outputs and rank == 0:
+            c2_last_ids = np.concatenate([b.column(0).to_numpy() for b in r2.batches]) if r2.batches else np.array([], np.int64)
         c2 = {"workload": C2_WORKLOAD, "value": rows_per_gpu * world / (dt2 / args.steps), "unit": "rows/s", "ms_per_step": 1000.0 * dt2 / args.steps,
               "selected_rows_per_gpu": sel, "kernel": "k_flat_filter", "kernel_ms": sum(k_ms2) / len(k_ms2),
               "algorithmic_bytes": r2.metrics["algorithmic_bytes"], "d2h_bytes_per_step": r2.metrics["d2h_bytes"],
@@ -528,7 +584,7 @@ def main():
             for _ in range(2):
                 r2e = prov2e.scan(filters=flt)
             barrier()
-            k = max(3, min(args.steps, 10))
+            k = args.steps
             t_a = time.perf_counter()
             for _ in range(k):
                 r2e = prov2e.scan(filters=flt)
@@ -623,6 +679,9 @@ def main():
     line["step_ms_quantiles"] = {"p10": q[len(q) // 10], "p50": q[len(q) // 2], "p90": q[(len(q) * 9) // 10], "max": q[-1]}
     line["step_ms"] = [round(x, 3) for x in step_ms]      # rank 0's wall time of every timed step, in order
     line["checks"] = checks
+    if args.dump_outputs:
+        lens = dump_outputs(args.dump_outputs, c4_last, c2_last_ids)
+        print(f"[bench] --dump-outputs: {lens} -> {args.dump_outputs}", file=sys.stderr)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier(group=gloo)
