@@ -200,8 +200,19 @@ struct DevPlan {
   uint32_t replicas;           // accumulator table copies in global memory; CTA b adds into copy b % replicas (merged by k_acc_reduce)
   uint32_t smem_share;         // of every 8 consumer warps of k_flat_agg, how many keep hot slots in shared memory (the rest use L2)
   uint32_t f64_global;         // 1: f64 SUM / AVG cells always go to L2 (no native shared-memory f64 atomic)
+  uint32_t f64_smem;           // 1: f64 SUM / AVG of every hot slot in shared memory (CAS loop); 0: only the per-lane cells, the
+                               // other hot slots send them to L2 (native reduction)
   uint32_t hashed;             // 1: the key space is wider than the dense table: group cells are found through DevScanArgs.hkeys
   uint32_t hmask;              // hashed: table capacity - 1 (nslots == capacity)
+  // flat aggregate kernel, shared-memory hot table: planes rows, acc[0 .. n_acc), nn[0 .. n_nn) as in the global table, but
+  // not all 8 bytes wide.  The rows and nn planes and the narrow MIN / MAX planes hold 4-byte cells; hot_off is each plane's
+  // byte offset inside the hot table (8-byte planes first, so every cell is aligned to its width)
+  uint32_t hot_off[1 + 2 * kMaxAggs];
+  uint32_t hot_cell_bytes;     // bytes of one hot cell over all planes
+  uint32_t acc_narrow;         // bit a: acc[a] is an Int64 MIN / MAX whose hot cells hold u32 offsets from acc_base[a]
+                               // (MIN: v - base, empty 0xffffffff; MAX: v - base + 1, empty 0).  A value outside
+                               // [base, base + 2^32 - 2] updates the global 8-byte cell instead
+  int64_t acc_base[kMaxAggs];
 };
 
 // Accumulator table layout (device, 8-byte cells, struct of arrays over nslots):

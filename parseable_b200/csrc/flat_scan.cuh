@@ -24,8 +24,8 @@
 //   surviving rows.  HBM traffic = encoded bytes once + 1 bit per row.
 // k_flat_agg<KR>: 31 consumer warps, one CTA per SM so that the hot part of the accumulator table
 //   (group slots < plan.hot_slots; group ids are numbered hot-first; the very hottest own a cell per
-//   lane) lives in shared memory next to the stages; cold slots go to L2 with fire-and-forget
-//   reductions.  Rows are dealt to threads interleaved (lane L of a warp takes row base + L):
+//   lane) lives in shared memory next to the stages, in cells as narrow as their updates allow; cold
+//   slots go to L2 with fire-and-forget reductions.  Rows are dealt to threads interleaved (lane L of a warp takes row base + L):
 //   neighbouring lanes share their index words, and 8-byte values are read in place from the flat
 //   store, fully coalesced.  Every pointer stays in ONE address space (a pointer that may be shared or
 //   global makes every access through it generic: that cost 20-25 % on both kernels before it was
@@ -695,8 +695,9 @@ k_flat_filter(const __grid_constant__ DevPlan plan, const __grid_constant__ Flat
 // made once per pass, outside the row loop.
 constexpr int kAggRowsMax = 8;   // k_flat_agg<KR>: KR = 8, 4, 2 rows per thread and slab
 
-// shared-memory cells are 8 bytes like the global ones; per-CTA partial counts and the low words of
-// partial sums are updated with native 32-bit atomics
+// Shared-memory cells are as narrow as their updates allow (plan.hot_off): counts are u32 (a CTA sees < 2^32 rows),
+// Int64 MIN / MAX whose range the footer statistics bound are u32 offsets, sums and f64 MIN / MAX keep 8 bytes.  The
+// flush widens every cell into the 8-byte global table.
 // `s` / `g`: the cell in the shared-memory table / in the global one, `hot` says which is meant.  Two pointers so
 // that each atomic is compiled for its address space (a pointer chosen at run time makes them generic: an address-space
 // test in front of every update, returning ATOM.E instead of RED for the cold cells).
@@ -719,6 +720,19 @@ __device__ __forceinline__ void cell_min_max(unsigned long long* s, unsigned lon
     if (is_min ? k >= cur : k <= cur) return;
     if (is_min) atomicMin(reinterpret_cast<long long*>(s), k);
     else atomicMax(reinterpret_cast<long long*>(s), k);
+  } else if (is_min) atomicMin(reinterpret_cast<long long*>(g), k);
+  else atomicMax(reinterpret_cast<long long*>(g), k);
+}
+// narrow Int64 MIN / MAX (plan.acc_narrow): one native 32-bit shared-memory atomic (ATOMS.MIN / MAX: no read, no CAS;
+// a plain read in front of it to skip rows that cannot improve the cell measured 1 % slower).
+// A value the statistics did not announce falls outside the window and goes to the global 8-byte cell `g` (the slot's
+// cell, also for a per-lane cell), which the flush merges with: the answer never depends on the statistics being right.
+constexpr uint64_t kNarrowSpan = 0xfffffffeull;   // offsets 0 .. kNarrowSpan (MAX stores offset + 1: 0 stays "empty")
+__device__ __forceinline__ void cell_min_max32(uint32_t* s, unsigned long long* g, bool hot, bool is_min, long long k, long long base) {
+  const uint64_t d = uint64_t(k) - uint64_t(base);
+  if (hot && d <= kNarrowSpan) {
+    if (is_min) atomicMin(s, uint32_t(d));
+    else atomicMax(s, uint32_t(d) + 1u);
   } else if (is_min) atomicMin(reinterpret_cast<long long*>(g), k);
   else atomicMax(reinterpret_cast<long long*>(g), k);
 }
@@ -757,18 +771,20 @@ k_flat_agg(const __grid_constant__ DevPlan plan, const __grid_constant__ FlatLay
   const uint32_t H = plan.hot_slots, nslots = plan.nslots, T = plan.lane_slots;
   const uint32_t Hs = H + 31u * T;   // cells per plane of the hot table
   const uint32_t cells = 1 + plan.n_acc + plan.n_nn;
-  unsigned long long* sacc = reinterpret_cast<unsigned long long*>(smem + L.acc);
+  uint8_t* const hot = smem + L.acc;
+  // plane p of the hot table, as 4-byte / 8-byte cells
+  auto hot32 = [&](uint32_t p) { return reinterpret_cast<uint32_t*>(hot + plan.hot_off[p]); };
+  auto hot64 = [&](uint32_t p) { return reinterpret_cast<unsigned long long*>(hot + plan.hot_off[p]); };
   // this CTA's copy of the global table (plan.replicas copies spread same-address traffic over L2; k_acc_reduce merges them)
   unsigned long long* gacc = a.acc + size_t(blockIdx.x % plan.replicas) * cells * nslots;
   flat_ctl_init(ctl, L.nstages, kAggConsumers / 32);
   for (uint32_t i = threadIdx.x; i < cells * Hs; i += kAggThreads) {
-    const uint32_t arr = i / Hs;
-    unsigned long long init = 0;
+    const uint32_t arr = i / Hs, c = i - arr * Hs;
     if (arr >= 1 && arr < 1 + plan.n_acc) {
       const uint8_t k = plan.acc_init[arr - 1];
-      init = k == 2 ? 0x7fffffffffffffffull : (k == 3 ? 0x8000000000000000ull : 0ull);
-    }
-    sacc[i] = init;
+      if ((plan.acc_narrow >> (arr - 1)) & 1u) hot32(arr)[c] = k == 2 ? 0xffffffffu : 0u;
+      else hot64(arr)[c] = k == 2 ? 0x7fffffffffffffffull : (k == 3 ? 0x8000000000000000ull : 0ull);
+    } else hot32(arr)[c] = 0u;   // rows, non-null counters
   }
   __syncthreads();
   const uint32_t S = plan.flat_slab_rows;
@@ -913,10 +929,11 @@ k_flat_agg(const __grid_constant__ DevPlan plan, const __grid_constant__ FlatLay
         else cell[i] = uint32_t(slot[i]) < Tw ? uint32_t(slot[i]) * 32u + lane : uint32_t(slot[i]) + 31u * Tw;
       }
       // ---- COUNT(*) cell ----
+      uint32_t* const srows = hot32(0);
 #pragma unroll
       for (int i = 0; i < KR; i++)
         if ((sel >> i) & 1u) {
-          if (cell[i] < Hw) atomicAdd(reinterpret_cast<uint32_t*>(&sacc[cell[i]]), 1u);   // a CTA sees < 2^32 rows: the low word never wraps
+          if (cell[i] < Hw) atomicAdd(&srows[cell[i]], 1u);
           else atomicAdd(&gadj[cell[i]], 1ull);
         }
       // ---- one pass per aggregate (NULL inputs contribute nothing) ----
@@ -934,10 +951,11 @@ k_flat_agg(const __grid_constant__ DevPlan plan, const __grid_constant__ FlatLay
         }
         if (ag.update_nn) {
           const uint32_t arr = 1 + plan.n_acc + ag.nn_slot;
+          uint32_t* const snn = hot32(arr);
 #pragma unroll
           for (int i = 0; i < KR; i++)
             if ((vsel >> i) & 1u) {
-              if (cell[i] < Hw) atomicAdd(reinterpret_cast<uint32_t*>(&sacc[arr * Hs + cell[i]]), 1u);
+              if (cell[i] < Hw) atomicAdd(&snn[cell[i]], 1u);
               else atomicAdd(&gadj[size_t(arr) * nslots + cell[i]], 1ull);
             }
         }
@@ -945,12 +963,15 @@ k_flat_agg(const __grid_constant__ DevPlan plan, const __grid_constant__ FlatLay
         const bool plain = c.fkind == FK_PLAIN8;
         const uint64_t* __restrict__ dict = reinterpret_cast<const uint64_t*>(a.flat + st.col[ag.col].dict8);
         const uint64_t* v8 = c.v8;
-        unsigned long long* scell = sacc + size_t(1 + ag.acc_slot) * Hs;
+        unsigned long long* scell = hot64(1 + ag.acc_slot);
         unsigned long long* gcell = gadj + size_t(1 + ag.acc_slot) * nslots;
         const bool f64 = ag.kind == DK_F64;
         const uint32_t fn = ag.fn;
-        // f64 sums have no native shared-memory atomic (a CAS loop): plan.f64_global sends them to L2
-        const uint32_t Hc = (plan.f64_global && (fn == AG_AVG || (fn == AG_SUM && f64))) ? 0u : Hw;
+        // f64 sums have no native shared-memory atomic (a CAS loop that retires one colliding lane per trip): only the
+        // per-lane cells, where the lanes of a warp never meet, keep them in shared memory; every other hot slot sends
+        // them to L2 as fire-and-forget reductions (plan.f64_smem: all hot slots, plan.f64_global: none)
+        const bool f64_add = fn == AG_AVG || (fn == AG_SUM && f64);
+        const uint32_t Hc = !f64_add ? Hw : plan.f64_global ? 0u : plan.f64_smem ? Hw : 32u * Tw;
         // the values first (all loads in flight together: a dictionary value is an L2 round trip), then the updates,
         // one straight-line loop per aggregate function
         uint64_t bits[KR];
@@ -977,17 +998,32 @@ k_flat_agg(const __grid_constant__ DevPlan plan, const __grid_constant__ FlatLay
           // MIN(x), MAX(x) next to each other: one pass over the values feeds both cells (the second aggregate of a
           // column never owns the non-null counter, so nothing else of its pass is left)
           const DevAgg& nx = plan.aggs[g + 1 < plan.naggs ? g + 1 : g];
-          const bool pair = g + 1 < plan.naggs && nx.col == ag.col && (nx.fn == AG_MIN || nx.fn == AG_MAX) && !nx.update_nn;
-          unsigned long long* scell2 = sacc + size_t(1 + nx.acc_slot) * Hs;
+          const bool narrow = (plan.acc_narrow >> ag.acc_slot) & 1u;   // decided per column: MIN and MAX of it agree
+          const bool pair = g + 1 < plan.naggs && nx.col == ag.col && (nx.fn == AG_MIN || nx.fn == AG_MAX) && !nx.update_nn &&
+                            narrow == (((plan.acc_narrow >> nx.acc_slot) & 1u) != 0);
           unsigned long long* gcell2 = gadj + size_t(1 + nx.acc_slot) * nslots;
           const bool is_min2 = nx.fn == AG_MIN;
+          if (narrow) {
+            uint32_t* s32 = hot32(1 + ag.acc_slot);
+            uint32_t* s32b = hot32(1 + nx.acc_slot);
+            const long long base = plan.acc_base[ag.acc_slot], base2 = plan.acc_base[nx.acc_slot];
 #pragma unroll
-          for (int i = 0; i < KR; i++)
-            if ((vsel >> i) & 1u) {
-              const long long k = f64 ? (long long)f64_order_key(bits[i]) : (long long)bits[i];
-              cell_min_max(scell + cell[i], gcell + cell[i], cell[i] < Hc, is_min, k);
-              if (pair) cell_min_max(scell2 + cell[i], gcell2 + cell[i], cell[i] < Hc, is_min2, k);
-            }
+            for (int i = 0; i < KR; i++)
+              if ((vsel >> i) & 1u) {
+                const uint32_t gc = cell[i] < 32u * Tw ? (cell[i] >> 5) + 31u * Tw : cell[i];   // the slot's global cell
+                cell_min_max32(s32 + cell[i], gcell + gc, cell[i] < Hc, is_min, (long long)bits[i], base);
+                if (pair) cell_min_max32(s32b + cell[i], gcell2 + gc, cell[i] < Hc, is_min2, (long long)bits[i], base2);
+              }
+          } else {
+            unsigned long long* scell2 = hot64(1 + nx.acc_slot);
+#pragma unroll
+            for (int i = 0; i < KR; i++)
+              if ((vsel >> i) & 1u) {
+                const long long k = f64 ? (long long)f64_order_key(bits[i]) : (long long)bits[i];
+                cell_min_max(scell + cell[i], gcell + cell[i], cell[i] < Hc, is_min, k);
+                if (pair) cell_min_max(scell2 + cell[i], gcell2 + cell[i], cell[i] < Hc, is_min2, k);
+              }
+          }
           if (pair) g++;
         }
       }
@@ -1004,15 +1040,22 @@ k_flat_agg(const __grid_constant__ DevPlan plan, const __grid_constant__ FlatLay
   // ---- flush the hot table ----
   __syncthreads();
   for (uint32_t cell = threadIdx.x; cell < Hs; cell += kAggThreads) {
-    const unsigned long long rows = sacc[cell];
+    const uint32_t rows = hot32(0)[cell];
     if (rows == 0) continue;
     const uint32_t slot = cell < 32u * T ? cell >> 5 : cell - 31u * T;
-    atomicAdd(&gacc[slot], rows);
-    for (uint32_t arr = 0; arr < plan.n_acc; arr++)
-      acc_merge(&gacc[(1 + arr) * nslots + slot], plan.acc_init[arr], sacc[(1 + arr) * Hs + cell]);
+    atomicAdd(&gacc[slot], (unsigned long long)rows);
+    for (uint32_t arr = 0; arr < plan.n_acc; arr++) {
+      const uint8_t how = plan.acc_init[arr];
+      unsigned long long* g = &gacc[(1 + arr) * nslots + slot];
+      if ((plan.acc_narrow >> arr) & 1u) {
+        const uint32_t v = hot32(1 + arr)[cell];
+        if (how == 2 ? v != 0xffffffffu : v != 0u)   // empty: every value of the slot went to the global cell (or was NULL)
+          acc_merge(g, how, uint64_t(plan.acc_base[arr]) + v - (how == 2 ? 0u : 1u));
+      } else acc_merge(g, how, hot64(1 + arr)[cell]);
+    }
     for (uint32_t k = 0; k < plan.n_nn; k++) {
-      const unsigned long long v = sacc[(1 + plan.n_acc + k) * Hs + cell];
-      if (v) atomicAdd(&gacc[(1 + plan.n_acc + k) * nslots + slot], v);
+      const uint32_t v = hot32(1 + plan.n_acc + k)[cell];
+      if (v) atomicAdd(&gacc[(1 + plan.n_acc + k) * nslots + slot], (unsigned long long)v);
     }
   }
 }

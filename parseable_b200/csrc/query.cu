@@ -1130,6 +1130,38 @@ void Query::run(const PqQueryDesc& d) {
   }
   plan.nslots = uint32_t(nslots64);
   const uint32_t cells = 1 + plan.n_acc + plan.n_nn;
+  // An Int64 MIN / MAX keeps 4-byte offsets from a base in the flat aggregate kernel's hot table when the footer
+  // statistics of every row group read bound the column to fewer than 2^32 - 1 values (one native shared-memory atomic per
+  // update instead of a read and a CAS loop).  Statistics that understate the range cost speed, never the answer: a value
+  // outside the window updates the global 8-byte cell (cell_min_max32).  PQB_AGG_WIDE_CELLS=1: 8-byte cells (A/B switch).
+  plan.acc_narrow = 0;
+  if (agg_kernel && !plan.hashed && !(getenv("PQB_AGG_WIDE_CELLS") && atoi(getenv("PQB_AGG_WIDE_CELLS")))) {
+    for (uint32_t a = 0; a < d.n_aggs; a++) {
+      const DevAgg& ag = plan.aggs[a];
+      if ((ag.fn != AG_MIN && ag.fn != AG_MAX) || ag.kind != DK_I64) continue;
+      int64_t vmin = INT64_MAX, vmax = INT64_MIN;
+      bool bounded = true;
+      for (uint32_t g = 0; g < nrg_table && bounded; g++) {
+        if (!rg_live[g]) continue;
+        const TableChunk& tc = table->row_groups[g].chunks[shape_cols[ag.col]];
+        if (!tc.present) continue;
+        const ColumnStats& st = tc.meta->stats;
+        if (st.null_count >= 0 && uint64_t(st.null_count) == uint64_t(tc.meta->num_values)) continue;   // all NULL: no values
+        if (!st.has_min || !st.has_max || st.min.size() != 8 || st.max.size() != 8) { bounded = false; break; }
+        int64_t mn, mx;
+        std::memcpy(&mn, st.min.data(), 8);
+        std::memcpy(&mx, st.max.data(), 8);
+        vmin = std::min(vmin, mn);
+        vmax = std::max(vmax, mx);
+      }
+      if (!bounded || vmin > vmax || uint64_t(vmax) - uint64_t(vmin) > kNarrowSpan) continue;
+      // the window [base, base + kNarrowSpan] must not wrap past INT64_MAX
+      plan.acc_base[ag.acc_slot] = std::min<int64_t>(vmin, INT64_MAX - int64_t(kNarrowSpan));
+      plan.acc_narrow |= 1u << ag.acc_slot;
+    }
+  }
+  plan.hot_cell_bytes = 4 * (1 + plan.n_nn);
+  for (uint32_t a = 0; a < plan.n_acc; a++) plan.hot_cell_bytes += ((plan.acc_narrow >> a) & 1u) ? 4 : 8;
 
   // ---- which kernels run ----
   (void)has_null_const;   // the flat kernels evaluate SQL three-valued logic, NULL literals included
@@ -1227,24 +1259,25 @@ void Query::run(const PqQueryDesc& d) {
       plan.hot_slots = 0;
     } else {
       // one CTA per SM: the hot part of the accumulator table next to the stages
-      const uint64_t full = plan.hashed ? 0 : uint64_t(plan.nslots) * cells * 8;   // hashed: no hot table in shared memory
+      const uint32_t cell_bytes = plan.hot_cell_bytes;
+      const uint64_t full = plan.hashed ? 0 : uint64_t(plan.nslots) * cell_bytes;   // hashed: no hot table in shared memory
       uint32_t krows = plan.hashed ? 4 : 8;   // the hashed instantiation exists for 4 rows per thread (64-bit slots: registers)
       if (const char* e = plan.hashed ? nullptr : getenv("PQB_AGG_KROWS")) krows = std::max(1, std::min(8, atoi(e)));   // experiment switch
       while (krows & (krows - 1)) krows &= krows - 1;
       while (krows > 1 && 2 * stage_bytes_for(kAggConsumers * krows) + std::min<uint64_t>(full, 96 * 1024) > avail) krows >>= 1;
       const uint32_t S = kAggConsumers * krows;
       FL.stage_bytes = stage_bytes_for(S);
-      if (2 * FL.stage_bytes + cells * 8 > avail) throw Error(PQ_ERR_UNSUPPORTED, "query needs more shared memory than one SM has");
+      if (2 * FL.stage_bytes + cell_bytes > avail) throw Error(PQ_ERR_UNSUPPORTED, "query needs more shared memory than one SM has");
       FL.nstages = 2;
       uint32_t left = avail - 2 * FL.stage_bytes;
       if (full + FL.stage_bytes <= left && FL.nstages < (uint32_t)kFlatStagesMax) { FL.nstages = 3; left -= FL.stage_bytes; }
       if (const char* e = getenv("PQB_AGG_STAGES")) {   // experiment switch: a deeper ring at the price of hot slots
         const uint32_t want = uint32_t(std::max(2, std::min(int(kFlatStagesMax), atoi(e))));
-        while (FL.nstages < want && left >= FL.stage_bytes + meta_stride + 64 * cells * 8) { FL.nstages++; left -= FL.stage_bytes + meta_stride; }
+        while (FL.nstages < want && left >= FL.stage_bytes + meta_stride + 64 * cell_bytes) { FL.nstages++; left -= FL.stage_bytes + meta_stride; }
       }
       // the hottest groups own a cell per lane (no same-address lanes inside a warp): 31 more cells each
-      const uint32_t cap = left / (cells * 8);
-      uint32_t T = 8;
+      const uint32_t cap = left / cell_bytes;
+      uint32_t T = 16;   // C4 with the narrow cells: 16 beats 8 by 2.4 %, 32 by 1 % more (profiles/probe_ab_summary_r3.md)
       if (const char* e = getenv("PQB_LANE_SLOTS")) T = uint32_t(std::max(0, atoi(e)));   // experiment switch
       if (const char* e = getenv("PQB_F64_GLOBAL")) if (atoi(e)) T = 0;   // that experiment sends hot f64 cells to L2 by SLOT: no per-lane cells
       T = std::min<uint32_t>(T, plan.nslots);
@@ -1255,10 +1288,20 @@ void Query::run(const PqQueryDesc& d) {
       if (const char* hs = plan.hashed ? nullptr : getenv("PQB_HOT_SLOTS")) plan.hot_slots = std::max(T, std::min<uint32_t>(plan.hot_slots, uint32_t(atoi(hs))));   // experiment switch
       plan.flat_slab_rows = S;
       plan.flat_krows = krows;
+      // hot table planes: the 8-byte ones first, so that every cell is aligned to its width
+      const uint32_t Hs = plan.hot_slots + 31u * T;
+      uint32_t off = 0;
+      for (int pass = 0; pass < 2; pass++)
+        for (uint32_t p = 0; p < cells; p++) {
+          const bool w8 = p >= 1 && p <= plan.n_acc && !((plan.acc_narrow >> (p - 1)) & 1u);
+          if (w8 != (pass == 0)) continue;
+          plan.hot_off[p] = off;
+          off += Hs * (w8 ? 8u : 4u);
+        }
     }
     FL.stage0 = align_up(FL.meta0 + FL.nstages * meta_stride, 128);
     FL.acc = align_up(FL.stage0 + FL.nstages * FL.stage_bytes, 128);
-    FL.total = FL.acc + (agg_kernel ? (plan.hot_slots + 31u * plan.lane_slots) * cells * 8 : 0);
+    FL.total = FL.acc + (agg_kernel ? (plan.hot_slots + 31u * plan.lane_slots) * plan.hot_cell_bytes : 0);
     if (FL.total > ctx.smem_optin()) throw Error(PQ_ERR_UNSUPPORTED, "query needs more shared memory than one SM has");
   }
 
@@ -1295,10 +1338,16 @@ void Query::run(const PqQueryDesc& d) {
   plan.f64_global = 0;
   if (const char* e = getenv("PQB_SMEM_SHARE")) plan.smem_share = uint32_t(atoi(e));
   if (const char* e = getenv("PQB_F64_GLOBAL")) plan.f64_global = uint32_t(atoi(e));
+  plan.f64_smem = 0;
+  if (const char* e = getenv("PQB_F64_SMEM")) plan.f64_smem = uint32_t(atoi(e));   // A/B switch: f64 sums of every hot slot in shared memory
   if (agg_kernel) {
+    bool f64_add = false;   // an f64 SUM / AVG: the hot slots without per-lane cells send it to L2
+    for (uint32_t a = 0; a < plan.naggs; a++)
+      f64_add |= plan.aggs[a].fn == AG_AVG || (plan.aggs[a].fn == AG_SUM && plan.aggs[a].kind == DK_F64);
+    const bool f64_l2 = f64_add && !plan.f64_smem && plan.hot_slots > plan.lane_slots;
     // Cold group slots go to L2 with fire-and-forget reductions; L2 serialises same-address atomics, so the
     // table is kept in a few copies (CTA b adds into copy b mod replicas) as long as all copies stay L2 resident.
-    if (n_flat && (plan.hot_slots < plan.nslots || plan.smem_share < 8 || plan.f64_global)) {
+    if (n_flat && (plan.hot_slots < plan.nslots || plan.smem_share < 8 || plan.f64_global || f64_l2)) {
       const uint64_t tbytes = uint64_t(plan.nslots) * cells * 8;
       uint32_t r = uint32_t(std::min<uint64_t>(32, (48ull << 20) / std::max<uint64_t>(tbytes, 1)));
       if (const char* e = getenv("PQB_REPLICAS")) r = uint32_t(atoi(e));
